@@ -2,6 +2,7 @@
 """bench.py -- forward+backward frames/sec of the render path on BASELINE.json's headline config.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c5] [--quick]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config C3 of BASELINE.json): 2 M frosting-layer Gaussians bound to the prism cells of a ~1 M-face
@@ -26,7 +27,12 @@ Sub-blocks of the JSON line (N = 1 only, each with the shipped kernels): `dropin
 `frosting_train_step`, `dp_train_step` (+ `dp_check`).
 
 Timing: CUDA events around exactly K steps after W warm-up steps, barrier + synchronize on both sides, max over
-ranks.  Inputs are larger than L2 (472 MB of attributes are read per frame, 126 MB L2), no flush needed.
+ranks.
+
+--dump-outputs DIR writes, right after the timed steps, what the last timed step handed its caller as DIR/<name>.npy
+(float32): the image, and radii and every gradient at a fixed seeded sample of Gaussian rows (DUMP_ROWS, the same on
+every run).  Scene, cameras and cotangents are seeded, so two builds run with the same arguments can be compared
+output for output.  Inputs are larger than L2 (472 MB of attributes are read per frame, 126 MB L2), no flush needed.
 """
 import argparse
 import json
@@ -48,6 +54,8 @@ from frosting_b200 import camera_batch as cb   # noqa: E402  (imports no native 
 METRIC = "fwd+bwd frames/sec @2M Gaussians 1080p"
 UNIT = "frames/s"
 DP_LEG_TIMEOUT_S = 240
+DUMP_ROWS = 65536
+DUMP_MAX_BYTES = 64 << 20
 RING_RADIUS = float(os.environ.get("FB200_RING_RADIUS", str(cb.RING_RADIUS)))
 
 
@@ -156,6 +164,7 @@ class ReferenceBatch:
             m3, op, sh, sc, ro = m3[render_mask], op[render_mask], sh[render_mask], sc[render_mask], ro[render_mask]
         means2D = torch.zeros_like(m3, requires_grad=True)
         color, radii = self.refdgr.RefRasterize.apply(m3, means2D, sh, op, sc, ro, rs)
+        self.last = dict(color=color, radii=radii, means2D=means2D)
         if self.loss_mode == "l1_dssim":
             from frosting_b200.loss import torch_reference     # restates frosting_utils/loss_utils.py:17-63 verbatim
             loss = torch_reference(color, self.gt[i], 0.2)
@@ -421,6 +430,28 @@ def dp_oracle_check(device, world, rank):
     return out
 
 
+def dump_outputs(step, out_dir, P):
+    """The last frame's image, and its radii and gradients at DUMP_ROWS fixed rows, as float32 .npy files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.randperm(P, generator=torch.Generator().manual_seed(0))[:min(P, DUMP_ROWS)].sort().values
+    arrays = {"color": step.last["color"]}
+    tensors = dict(getattr(step, "leaves", None) or step.params)
+    if step.last.get("means2D") is not None:
+        tensors["means2D"] = step.last["means2D"]
+    per_row = {"radii": step.last["radii"], **{"grad_" + k: v.grad for k, v in tensors.items() if v.grad is not None}}
+    for k, v in per_row.items():
+        # a gathered call (boolean-masked inputs) returns fewer rows than the scene has: sample only rows it has
+        arrays[k] = v[rows[rows < v.shape[0]].to(v.device)]
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}")
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    log(f"[bench] wrote {len(arrays)} arrays ({total / 2**20:.1f} MB) to {out_dir}")
+
+
 def make_step(impl, wl, device, **kw):
     if impl == "ours":
         return cb.CameraBatch(wl, device, **kw)
@@ -492,6 +523,8 @@ def main():
     ap.add_argument("--with-dp", action="store_true", help="with --quick: also run the data-parallel training leg")
     ap.add_argument("--frame", default="raster", choices=["raster", "frosting"],
                     help="developer runs: time the frame from Frosting's parameters (frosting_render) as the main loop")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE JSON line: route fd 1 to stderr for the whole run (NCCL / C libraries print their
@@ -532,6 +565,8 @@ def main():
     secs, t0, t1 = timed_loop(step, wl, device, args.steps, args.warmup, world, e2e=False, count_launches=ours)
     clocks = sampler.stop(t0, t1) if sampler else None
     launches_timed = timed_loop.launches if ours else 0   # kernels of libfrosting_b200.so launched inside the timed region
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step, args.dump_outputs, wl["P"])
     value = world * args.steps / secs
 
     e2e_value = None

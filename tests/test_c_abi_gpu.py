@@ -9,8 +9,7 @@ import torch
 import frosting_b200 as fb
 from frosting_b200 import _lib
 from frosting_b200._lib import Params, Inputs, Workspace, Grads
-from oracle import refdgr
-from tests.util import scene, rel_err_stats
+from tests.util import scene, rel_err_stats, golden_case, check_inputs, check_forward, ours_forward_fields
 
 pytestmark = pytest.mark.gpu
 
@@ -87,17 +86,17 @@ def test_one_phase_forward_overflow_protocol_and_backward(cuda_device):
     assert L.fb200_backward(C.byref(prm), C.byref(inp), C.byref(ws), _p(radii), _p(cot), C.byref(bad), stream) == -1
 
 
-@pytest.mark.skipif(not refdgr.available(), reason="oracle/_ref not built")
+def many_tiles_scene(device):
+    P, W, H, D = 40_000, 2608, 1712, 1
+    cam, g, rs = scene(P, W, H, 12, D, device, 0.0)
+    return P, rs, g
+
+
 def test_frame_with_more_tiles_than_the_scan_stages(cuda_device):
     """2608 x 1712 = 163 x 107 = 17 441 tiles > 10 240: the tile scan reads its counts from global memory."""
-    dev = cuda_device
-    P, W, H, D = 40_000, 2608, 1712, 1
-    cam, g, rs = scene(P, W, H, 12, D, dev, 0.0)
-    kw = dict(shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], **kw)
-    st = fb.forward_with_state(rs, g["means3D"], g["opacities"], **kw)
-    assert st["num_rendered"] == ref["num_rendered"]
-    assert torch.equal(st["radii"], ref["radii"])
-    assert torch.equal(st["point_list"], refdgr.binning_views(ref["binning"], ref["num_rendered"])["point_list"])
-    assert torch.equal(st["n_contrib"], refdgr.img_views(ref["img"], H, W)["n_contrib"])
-    assert (st["color"] - ref["color"]).abs().max().item() <= 1e-4
+    P, rs, g = many_tiles_scene(cuda_device)
+    case = golden_case("cabi_many_tiles")
+    check_inputs(case, *(g[k] for k in ("means3D", "opacities", "shs", "scales", "rotations")))
+    st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    f = ours_forward_fields(st)
+    check_forward(case, {k: f[k] for k in ("num_rendered", "radii", "point_list", "n_contrib", "color")})

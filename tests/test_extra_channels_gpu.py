@@ -1,18 +1,14 @@
 """Row f4: extra feature channels blended in the same traversal == the reference's SECOND rasterizer pass with the
 features as colors_precomp (frosting_scene/sugar_model.py:2343-2387), forward and backward."""
-import numpy as np
 import pytest
 import torch
 
 import frosting_b200 as fb
-from oracle import refdgr
-from tests.util import scene, rel_err_stats
+from tests.util import scene, golden_case, check_inputs, check_forward, check_grad
 
 pytestmark = pytest.mark.gpu
 
-
-def _ref_available():
-    return refdgr.available()
+PARAMS = [(3, 0.0), (3, 0.25), (1, 0.0), (2, 1.0)]
 
 
 def _features(P, E, cam_like_depth, gen, device):
@@ -22,27 +18,27 @@ def _features(P, E, cam_like_depth, gen, device):
     return f.to(device)
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("E,bg_e", [(3, 0.0), (3, 0.25), (1, 0.0), (2, 1.0)])
-def test_extra_pass_matches_second_reference_pass(E, bg_e, cuda_device):
-    dev = cuda_device
+def extra_inputs(E, device):
     P, W, H, D = 60_000, 400, 304, 3
-    cam, g, rs = scene(P, W, H, 21, D, dev, 0.5)
+    cam, g, rs = scene(P, W, H, 21, D, device, 0.5)
     gen = torch.Generator().manual_seed(8)
-    feats = _features(P, E, None, gen, dev)
-    cot_c = torch.randn(3, H, W, generator=gen).to(dev)
-    cot_e = torch.randn(E, H, W, generator=gen).to(dev)
-    bg_extra = torch.full((E,), bg_e, device=dev)
+    feats = _features(P, E, None, gen, device)
+    cot_c = torch.randn(3, H, W, generator=gen).to(device)
+    cot_e = torch.randn(E, H, W, generator=gen).to(device)
+    return rs, g, feats, cot_c, cot_e
 
-    # reference: pass 1 (SH colours), pass 2 (features as colors_precomp, padded to 3 channels)
+
+@pytest.mark.parametrize("E,bg_e", PARAMS)
+def test_extra_pass_matches_second_reference_pass(E, bg_e, cuda_device):
+    """The reference's outputs (tests/golden/make_ref_golden.py): pass 1 with the SH colours, pass 2 with the features
+    as colors_precomp padded to 3 channels over a background of bg_e; gradients are the sum of both passes'."""
+    dev = cuda_device
+    rs, g, feats, cot_c, cot_e = extra_inputs(E, dev)
+    P, H, W = feats.shape[0], rs.image_height, rs.image_width
+    bg_extra = torch.full((E,), bg_e, device=dev)
     kw = dict(scales=g["scales"], rotations=g["rotations"])
-    ref1 = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], **kw)
-    f3 = torch.zeros(P, 3, device=dev); f3[:, :E] = feats
-    rs2 = rs._replace(bg=torch.full((3,), bg_e, device=dev))
-    ref2 = refdgr.forward(rs2, g["means3D"], g["opacities"], colors_precomp=f3, **kw)
-    cot2 = torch.zeros(3, H, W, device=dev); cot2[:E] = cot_e
-    rb1 = refdgr.backward(rs, ref1, g["means3D"], cot_c, shs=g["shs"], **kw)
-    rb2 = refdgr.backward(rs2, ref2, g["means3D"], cot2, colors_precomp=f3, **kw)
+    case = golden_case(f"extra_E{E}_bg{bg_e:g}")
+    check_inputs(case, *(g[k] for k in ("means3D", "opacities", "shs", "scales", "rotations")), feats, cot_c, cot_e)
 
     leaves = {k: g[k].clone().requires_grad_(True) for k in ("means3D", "opacities", "shs", "scales", "rotations")}
     fl = feats.clone().requires_grad_(True)
@@ -51,24 +47,17 @@ def test_extra_pass_matches_second_reference_pass(E, bg_e, cuda_device):
         means3D=leaves["means3D"], means2D=m2, opacities=leaves["opacities"], shs=leaves["shs"],
         scales=leaves["scales"], rotations=leaves["rotations"], extra_features=fl, extra_background=bg_extra)
     assert extra.shape == (E, H, W)
-    assert torch.equal(radii, ref1["radii"])
     # colour is untouched by the extension: bit-identical to the colour-only call
     c0, _ = fb.GaussianRasterizer(rs)(means3D=g["means3D"], means2D=torch.zeros(P, 3, device=dev),
                                       opacities=g["opacities"], shs=g["shs"], **kw)
     assert torch.equal(color.detach().view(torch.int32), c0.view(torch.int32))
-    assert (extra.detach() - ref2["color"][:E]).abs().max().item() <= 2e-6 * max(1.0, float(feats.abs().max()))
+    check_forward(case, {"radii": radii, "color": extra.detach()}, color_tol=2e-6 * max(1.0, float(feats.abs().max())))
 
     ((color * cot_c).sum() + (extra * cot_e).sum()).backward()
-    want = {k: rb1[k] + rb2[k] for k in ("means3D", "means2D", "opacities", "scales", "rotations")}
     got = dict(means3D=leaves["means3D"].grad, means2D=m2.grad, opacities=leaves["opacities"].grad,
-               scales=leaves["scales"].grad, rotations=leaves["rotations"].grad)
-    for k in want:
-        m, frac = rel_err_stats(got[k], want[k])
-        assert m <= 1e-3 and frac <= 5e-3, (k, m, frac)
-    m, frac = rel_err_stats(leaves["shs"].grad, rb1["sh"])
-    assert m <= 1e-3 and frac <= 5e-3, ("sh", m, frac)
-    m, frac = rel_err_stats(fl.grad, rb2["colors"][:, :E])
-    assert m <= 1e-3 and frac <= 5e-3, ("features", m, frac)
+               scales=leaves["scales"].grad, rotations=leaves["rotations"].grad, sh=leaves["shs"].grad, features=fl.grad)
+    for k, v in got.items():
+        check_grad(case, k, v, radii, frac_bar=5e-3, tag=f"extra E{E}")
     assert torch.equal(fl.grad[radii <= 0], torch.zeros_like(fl.grad[radii <= 0]))
 
 

@@ -1,57 +1,63 @@
-"""Pins the C oracle (oracle/raster_oracle.c) to the UNMODIFIED compiled reference (oracle/_ref), and the CUDA
-mesh prepass to its C restatement.  Runs on the GPU box only because the reference is CUDA code."""
+"""Pins the C oracle (oracle/raster_oracle.c) to the UNMODIFIED reference, whose outputs for these inputs are recorded in
+tests/golden/ref_outputs.npz (tests/golden/make_ref_golden.py), and the CUDA mesh prepass to its C restatement."""
 import numpy as np
 import pytest
 import torch
 
 import frosting_b200 as fb
 from frosting_b200 import scenes
-from oracle import cpu, refdgr
-from tests.util import scene
+from oracle import cpu
+from tests.util import scene, golden_case, check_inputs, check_forward, grad_sample_index, spread
 
 pytestmark = pytest.mark.gpu
 
+CONFIGS = [(6000, 200, 136, 31, 3, 0.0), (4000, 96, 64, 32, 1, 1.0), (10_000, 256, 256, 1235, 0, 0.0)]
+IDS = ["D3", "D1_bg1", "C1"]
+FWD_FIELDS = ("radii", "depth", "means2D", "conic", "rgb", "cov3D", "touched", "num_rendered", "point_list", "keys",
+              "ranges", "n_contrib")
+GRADS = ("means3D", "means2D", "sh", "opacities", "scales", "rotations", "colors", "cov3D")
+COLOR_SAMPLE = 1024
 
-@pytest.mark.skipif(not refdgr.available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("cfg", [(6000, 200, 136, 31, 3, 0.0), (4000, 96, 64, 32, 1, 1.0), (10_000, 256, 256, 1235, 0, 0.0)],
-                         ids=["D3", "D1_bg1", "C1"])
+
+def cotangent(H, W, device):
+    return torch.randn(3, H, W, generator=torch.Generator().manual_seed(1)).to(device)
+
+
+@pytest.mark.parametrize("cfg", CONFIGS, ids=IDS)
 def test_c_oracle_matches_compiled_reference(cfg, cuda_device):
     P, W, H, seed, D, bg = cfg
     cam, g, rs = scene(P, W, H, seed, D, cuda_device, bg)
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    cot = cotangent(H, W, cuda_device)
+    case = golden_case("oracle_" + IDS[CONFIGS.index(cfg)])
+    check_inputs(case, *(g[k] for k in ("means3D", "opacities", "shs", "scales", "rotations")), cot)
     A = {k: v.cpu().numpy() for k, v in g.items()}
     o = cpu.forward(rs, A["means3D"], A["opacities"], shs=A["shs"], scales=A["scales"], rots=A["rotations"])
-    gv = refdgr.geom_views(ref["geom"], P)
-    R = ref["num_rendered"]
-    vis = (ref["radii"] > 0).cpu().numpy()
-    # integer-determining stage: bit-exact on the CPU as well
-    assert np.array_equal(o["pre"]["radii"], ref["radii"].cpu().numpy())
-    assert np.array_equal(o["pre"]["depths"][vis].view(np.int32), gv["depths"].cpu().numpy()[vis].view(np.int32))
-    assert np.array_equal(o["pre"]["xy"][vis].view(np.int32), gv["means2D"].cpu().numpy()[vis].view(np.int32))
-    assert np.array_equal(o["pre"]["conic_opacity"][vis].view(np.int32), gv["conic_opacity"].cpu().numpy()[vis].view(np.int32))
-    assert np.array_equal(o["pre"]["rgb"][vis].view(np.int32), gv["rgb"].cpu().numpy()[vis].view(np.int32))
-    assert np.array_equal(o["pre"]["cov3D"][vis].view(np.int32), gv["cov3D"].cpu().numpy()[vis].view(np.int32))
-    assert np.array_equal(o["pre"]["tiles_touched"][vis].astype(np.int32), gv["tiles_touched"].cpu().numpy()[vis])
-    assert o["binned"]["num_rendered"] == R
-    bv = refdgr.binning_views(ref["binning"], R)
-    assert np.array_equal(o["binned"]["point_list"].astype(np.int32), bv["point_list"].cpu().numpy())
-    assert np.array_equal(o["binned"]["keys"].astype(np.int64), bv["point_list_keys"].cpu().numpy())
-    iv = refdgr.img_views(ref["img"], H, W)
-    assert np.array_equal(o["binned"]["ranges"].astype(np.int32), iv["ranges"].cpu().numpy())
-    # blend: host expf differs from libdevice's by ~2 ulp, so allow a handful of threshold flips
-    nc_ref = iv["n_contrib"].cpu().numpy()
+    vis = o["pre"]["radii"] > 0
+    pre = o["pre"]
+    # integer-determining stage and binning: bit-exact on the CPU as well
+    check_forward(case, dict(
+        radii=pre["radii"], depth=pre["depths"][vis].view(np.int32), means2D=pre["xy"][vis].view(np.int32),
+        conic=pre["conic_opacity"][vis].view(np.int32), rgb=pre["rgb"][vis].view(np.int32),
+        cov3D=pre["cov3D"][vis].view(np.int32), touched=pre["tiles_touched"][vis],
+        num_rendered=o["binned"]["num_rendered"], point_list=o["binned"]["point_list"], keys=o["binned"]["keys"],
+        ranges=o["binned"]["ranges"]))
+    # blend: host expf differs from libdevice's by ~2 ulp, so allow a handful of threshold flips.  The reference's
+    # per-pixel counts are stood in for by ours, which must equal them bit for bit.
+    st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    check_forward(case, {"n_contrib": st["n_contrib"]})
+    nc_ref = st["n_contrib"].cpu().numpy()
     assert (o["n_contrib"].astype(np.int32) != nc_ref).mean() < 1e-3
-    err = np.abs(o["color"] - ref["color"].cpu().numpy())
+    err = np.abs(o["color"].reshape(-1)[spread(o["color"].size, COLOR_SAMPLE)] - case["color"])
     assert np.quantile(err, 0.999) <= 1e-5 and err.max() <= 5e-3
     # backward (oracle accumulates in fp64, the reference with unordered float atomics)
-    cot = torch.randn(3, H, W, generator=torch.Generator().manual_seed(1)).to(cuda_device)
-    rb = refdgr.backward(rs, ref, g["means3D"], cot, shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
     ob = cpu.backward(rs, o, A["means3D"], cot.cpu().numpy(), shs=A["shs"], scales=A["scales"], rots=A["rotations"])
-    for k_o, k_r in (("means3D", "means3D"), ("means2D", "means2D"), ("sh", "sh"), ("opacities", "opacities"),
-                     ("scales", "scales"), ("rotations", "rotations"), ("colors", "colors"), ("cov3D", "cov3D")):
-        a, b = ob[k_o].astype(np.float64).ravel(), rb[k_r].cpu().numpy().astype(np.float64).ravel()
-        scale = max(np.abs(b).max(), 1e-30)
-        assert np.abs(a - b).max() / scale <= 2e-3, (k_o, np.abs(a - b).max() / scale)
+    radii = torch.from_numpy(pre["radii"])
+    for k in GRADS:
+        a = torch.from_numpy(ob[k])
+        mine = a.reshape(-1)[grad_sample_index(a, radii)].double().numpy()
+        scale = max(float(case[k + ".stats"][0]), 1e-30)
+        assert np.abs(mine - case[k + ".sample"]).max() / scale <= 2e-3, (k, np.abs(mine - case[k + ".sample"]).max() / scale)
+        assert abs(np.abs(ob[k]).max() - scale) <= 2e-3 * scale, (k, np.abs(ob[k]).max(), scale)
 
 
 def test_mesh_prepass_cuda_matches_c_restatement(cuda_device):

@@ -1,13 +1,13 @@
-"""GPU parity: frosting_b200 (through its C ABI) against the UNMODIFIED reference rasterizer compiled
-from /root/reference into oracle/_ref (SURVEY.md section 8c).  Integer / index work bit-exact, forward
-colour <= 1e-4 abs, gradients <= 1e-3 relative (tests/util.py::rel_err_stats)."""
+"""GPU parity: frosting_b200 (through its C ABI) against the UNMODIFIED reference rasterizer, whose outputs for these
+inputs are recorded in tests/golden/ref_outputs.npz (tests/golden/make_ref_golden.py; SURVEY.md section 8c).
+Integer / index work bit-exact, forward colour <= 1e-4 abs, gradients <= 1e-3 relative (tests/util.py::rel_err_stats)."""
 import pytest
 import torch
 
 import frosting_b200 as fb
 from frosting_b200 import rasterizer as fbr
-from oracle import refdgr
-from tests.util import scene, rel_err_stats
+from oracle import cpu
+from tests.util import scene, rel_err_stats, golden_case, check_inputs, check_forward, check_grad, ours_forward_fields
 
 pytestmark = pytest.mark.gpu
 
@@ -18,93 +18,58 @@ CONFIGS = [
     (200_000, 803, 597, 11, 2, 0.0),       # W, H not multiples of 16
     (500_000, 800, 800, 1236, 3, 0.0),     # BASELINE config 2
 ]
+KEYS = ("means3D", "opacities", "shs", "scales", "rotations")
+FWD_FIELDS = ("num_rendered", "radii", "depth", "touched", "means2D", "conic", "rgb", "clamped", "ranges", "point_list",
+              "key_depth", "key_index", "n_contrib", "final_T", "color")
+LIST_FIELDS = ("num_rendered", "point_list", "n_contrib", "color")
 
 
-def _ref_available():
-    return refdgr.available()
+def _id(c):
+    return f"P{c[0]}_{c[1]}x{c[2]}_D{c[4]}"
 
 
-def run_both(P, W, H, seed, D, bg, device):
-    cam, g, rs = scene(P, W, H, seed, D, device, bg)
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
-    st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"],
-                               rotations=g["rotations"])
-    return cam, g, rs, ref, st
+def _fields(st, names):
+    f = ours_forward_fields(st)
+    return {k: f[k] for k in names}
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("cfg", CONFIGS, ids=lambda c: f"P{c[0]}_{c[1]}x{c[2]}_D{c[4]}")
+def cotangent(H, W, device):
+    return torch.randn(3, H, W, generator=torch.Generator().manual_seed(99)).to(device)
+
+
+@pytest.mark.parametrize("cfg", CONFIGS, ids=_id)
 def test_forward_bit_exact_vs_reference(cfg, cuda_device):
     P, W, H, seed, D, bg = cfg
-    cam, g, rs, ref, st = run_both(*cfg, cuda_device)
-    gv = refdgr.geom_views(ref["geom"], P)
-    R = ref["num_rendered"]
-    bv = refdgr.binning_views(ref["binning"], R)
-    iv = refdgr.img_views(ref["img"], H, W)
-    vis = ref["radii"] > 0
-
-    # per-Gaussian integers and integer-determining floats: bit-exact
-    assert torch.equal(st["radii"], ref["radii"]), f"radii mismatches: {(st['radii'] != ref['radii']).sum().item()}"
-    assert st["num_rendered"] == R
-    rect = st["rect"]
-    minx, miny = rect[:, 0] & 0xffff, (rect[:, 0] >> 16) & 0xffff
-    maxx, maxy = rect[:, 1] & 0xffff, (rect[:, 1] >> 16) & 0xffff
-    touched = (maxx - minx) * (maxy - miny)
-    assert torch.equal(touched[vis], gv["tiles_touched"][vis])
-    assert torch.equal(st["depth"][vis].view(torch.int32), gv["depths"][vis].view(torch.int32)), "depth bits"
-    rec = st["rec"]
-    assert torch.equal(rec[vis][:, 0:2].contiguous().view(torch.int32), gv["means2D"][vis].view(torch.int32)), "means2D bits"
-    mine_co = torch.stack([rec[:, 2], rec[:, 3], rec[:, 4], rec[:, 5]], 1)
-    assert torch.equal(mine_co[vis].view(torch.int32), gv["conic_opacity"][vis].view(torch.int32)), "conic/opacity bits"
-    mine_rgb = torch.stack([rec[:, 6], rec[:, 7], rec[:, 8]], 1)
-    assert torch.equal(mine_rgb[vis].view(torch.int32), gv["rgb"][vis].view(torch.int32)), "SH colour bits"
-    cl = st["clamped"]
-    mine_cl = torch.stack([cl & 1, (cl >> 1) & 1, (cl >> 2) & 1], 1)
-    assert torch.equal(mine_cl[vis], gv["clamped"][vis])
-
-    # binning: ranges, sorted order, keys
-    assert torch.equal(st["ranges"], iv["ranges"]), "tile ranges"
-    assert torch.equal(st["point_list"], bv["point_list"]), \
-        f"point_list mismatches: {(st['point_list'] != bv['point_list']).sum().item()} of {R}"
-    # reference key = tile<<32 | depth_bits; ours = depth_bits<<32 | idx, per tile
-    ref_depth_bits = bv["point_list_keys"] & 0xffffffff
-    assert torch.equal(st["keys"] >> 32, ref_depth_bits)
-    assert torch.equal((st["keys"] & 0xffffffff).int(), bv["point_list"])
-
-    # blend: per-pixel integer state exact, colour within 1e-4 abs
-    assert torch.equal(st["n_contrib"], iv["n_contrib"]), \
-        f"n_contrib mismatches: {(st['n_contrib'] != iv['n_contrib']).sum().item()}"
-    assert torch.equal(st["final_T"].view(torch.int32), iv["accum_alpha"].view(torch.int32)), "final_T bits"
-    err = (st["color"] - ref["color"]).abs().max().item()
-    assert err <= 1e-4, f"forward colour max abs err {err}"
+    cam, g, rs = scene(P, W, H, seed, D, cuda_device, bg)
+    case = golden_case("parity_fwd_" + _id(cfg))
+    check_inputs(case, *(g[k] for k in KEYS))
+    st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"],
+                               rotations=g["rotations"])
+    # per-Gaussian integers and integer-determining floats, binning (ranges, sorted order, keys), per-pixel integer
+    # state: bit-exact; colour within 1e-4 abs.  Reference key = tile<<32 | depth_bits; ours = depth_bits<<32 | idx.
+    check_forward(case, _fields(st, FWD_FIELDS))
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("cfg", CONFIGS[:3], ids=lambda c: f"P{c[0]}_{c[1]}x{c[2]}_D{c[4]}")
+@pytest.mark.parametrize("cfg", CONFIGS[:3], ids=_id)
 def test_backward_vs_reference(cfg, cuda_device):
     P, W, H, seed, D, bg = cfg
     cam, g, rs = scene(P, W, H, seed, D, cuda_device, bg)
-    gen = torch.Generator().manual_seed(99)
-    cot = torch.randn(3, H, W, generator=gen).to(cuda_device)
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
-    rb = refdgr.backward(rs, ref, g["means3D"], cot, shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
-    rb2 = refdgr.backward(rs, ref, g["means3D"], cot, shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    cot = cotangent(H, W, cuda_device)
+    case = golden_case("parity_bwd_" + _id(cfg))
+    check_inputs(case, *(g[k] for k in KEYS), cot)
 
-    leaves = {k: g[k].clone().requires_grad_(True) for k in ("means3D", "opacities", "shs", "scales", "rotations")}
+    leaves = {k: g[k].clone().requires_grad_(True) for k in KEYS}
     means2D = torch.zeros(P, 3, device=cuda_device, requires_grad=True)
     color, radii = fb.GaussianRasterizer(rs)(
         means3D=leaves["means3D"], means2D=means2D, opacities=leaves["opacities"], shs=leaves["shs"],
         scales=leaves["scales"], rotations=leaves["rotations"])
     (color * cot).sum().backward()
+    check_forward(case, {"radii": radii})
     mine = dict(means3D=leaves["means3D"].grad, means2D=means2D.grad, sh=leaves["shs"].grad,
                 opacities=leaves["opacities"].grad, scales=leaves["scales"].grad, rotations=leaves["rotations"].grad)
     for k, v in mine.items():
-        assert v is not None and v.shape == rb[k].shape, k
-        m, frac = rel_err_stats(v, rb[k])
-        m0, frac0 = rel_err_stats(rb2[k], rb[k])   # the reference's own atomic-order noise
-        print(f"{k}: max err/scale {m:.3e} (ref self-noise {m0:.3e}), frac elem rel>1e-3 {frac:.3e} (ref {frac0:.3e})")
-        assert m <= 1e-3, f"{k}: max err relative to scale {m}"
-        assert frac <= max(2e-3, 3 * frac0), f"{k}: {frac} of significant elements differ by >1e-3 rel"
+        assert v is not None and v.shape == (means2D.shape if k == "means2D" else g["shs" if k == "sh" else k].shape), k
+        check_grad(case, k, v, radii, tag=_id(cfg))
     assert torch.equal(means2D.grad[:, 2], torch.zeros_like(means2D.grad[:, 2]))
 
 
@@ -125,37 +90,43 @@ def test_subtile_culling_is_output_neutral(cfg, cuda_device):
     assert torch.equal(a["final_T"].view(torch.int32), b["final_T"].view(torch.int32))
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
+def precomp_inputs(device):
+    """Inputs of the colors_precomp + cov3D_precomp case.  The covariances are the C oracle's preprocess output, which is
+    bit-exact with the reference's geometry buffer (test_oracle_vs_ref_gpu.py), so both sides see the covariance the
+    reference derives from these scales / rotations; culled rows get a small isotropic one."""
+    P, W, H = 50_000, 320, 240
+    cam, g, rs = scene(P, W, H, 5, 0, device, 0.5)
+    gen = torch.Generator().manual_seed(3)
+    colors = torch.rand(P, 3, generator=gen).to(device)
+    A = {k: g[k].cpu().numpy() for k in ("means3D", "opacities", "scales", "rotations")}
+    pre = cpu.preprocess(cpu.Camera(rs), A["means3D"], A["opacities"], colors_precomp=colors.cpu().numpy(),
+                         scales=A["scales"], rots=A["rotations"])
+    cov = torch.from_numpy(pre["cov3D"]).to(device)
+    cov[torch.from_numpy(pre["radii"] <= 0).to(device)] = \
+        0.01 * torch.eye(3, device=device)[[0, 0, 0, 1, 1, 2], [0, 1, 2, 1, 2, 2]]
+    cot = torch.randn(3, H, W, generator=gen).to(device)
+    return rs, g, colors, cov, cot
+
+
 def test_precomputed_colour_and_covariance_path(cuda_device):
     """colors_precomp + cov3D_precomp branch (forward.cu:204-215,243-249; depth/normal passes of
     sugar_model.py:2364-2375 use colors_precomp)."""
-    P, W, H = 50_000, 320, 240
-    cam, g, rs = scene(P, W, H, 5, 0, cuda_device, 0.5)
-    gen = torch.Generator().manual_seed(3)
-    colors = torch.rand(P, 3, generator=gen).to(cuda_device)
-    # covariance from the reference's own geometry buffer so both sides see identical inputs
-    ref0 = refdgr.forward(rs, g["means3D"], g["opacities"], colors_precomp=colors, scales=g["scales"], rotations=g["rotations"])
-    cov = refdgr.geom_views(ref0["geom"], P)["cov3D"].clone()
-    cov[ref0["radii"] <= 0] = 0.01 * torch.eye(3, device=cuda_device)[[0, 0, 0, 1, 1, 2], [0, 1, 2, 1, 2, 2]]
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], colors_precomp=colors, cov3D_precomp=cov)
+    rs, g, colors, cov, cot = precomp_inputs(cuda_device)
+    P = colors.shape[0]
+    case = golden_case("parity_precomp")
+    check_inputs(case, g["means3D"], g["opacities"], colors, cov, cot)
     st = fb.forward_with_state(rs, g["means3D"], g["opacities"], colors_precomp=colors, cov3D_precomp=cov)
-    assert torch.equal(st["radii"], ref["radii"])
-    assert torch.equal(st["point_list"], refdgr.binning_views(ref["binning"], ref["num_rendered"])["point_list"])
-    assert (st["color"] - ref["color"]).abs().max().item() <= 1e-4
-    cot = torch.randn(3, H, W, generator=gen).to(cuda_device)
-    rb = refdgr.backward(rs, ref, g["means3D"], cot, colors_precomp=colors, cov3D_precomp=cov)
+    check_forward(case, _fields(st, ("radii", "point_list", "color")))
     m3 = g["means3D"].clone().requires_grad_(True)
     col = colors.clone().requires_grad_(True)
     cv = cov.clone().requires_grad_(True)
     op = g["opacities"].clone().requires_grad_(True)
     m2 = torch.zeros(P, 3, device=cuda_device, requires_grad=True)
-    color, _ = fb.GaussianRasterizer(rs)(means3D=m3, means2D=m2, opacities=op, colors_precomp=col, cov3D_precomp=cv)
+    color, radii = fb.GaussianRasterizer(rs)(means3D=m3, means2D=m2, opacities=op, colors_precomp=col, cov3D_precomp=cv)
     (color * cot).sum().backward()
-    for name, mine, refg in (("means3D", m3.grad, rb["means3D"]), ("colors", col.grad, rb["colors"]),
-                             ("cov3D", cv.grad, rb["cov3D"]), ("opacities", op.grad, rb["opacities"]),
-                             ("means2D", m2.grad, rb["means2D"])):
-        m, frac = rel_err_stats(mine, refg)
-        assert m <= 1e-3 and frac <= 5e-3, (name, m, frac)
+    for name, mine in (("means3D", m3.grad), ("colors", col.grad), ("cov3D", cv.grad), ("opacities", op.grad),
+                       ("means2D", m2.grad)):
+        check_grad(case, name, mine, radii, frac_bar=5e-3, tag="precomp")
 
 
 def test_visibility_mask_equals_boolean_gather(cuda_device):
@@ -214,65 +185,67 @@ def test_edge_cases(cuda_device):
     vis = r.markVisible(g["means3D"])
     assert vis.dtype == torch.bool and torch.equal(vis, g["means3D"][:, 2] > 0.2)
     # a single huge Gaussian covering every tile (exercises long rects, single-instance tiles)
-    one = dict(means3D=torch.tensor([[0.0, 0.0, 3.0]], device=dev), opacities=torch.tensor([[0.9]], device=dev),
-               scales=torch.full((1, 3), 5.0, device=dev), rotations=torch.tensor([[1.0, 0, 0, 0]], device=dev),
-               shs=torch.ones(1, 16, 3, device=dev))
+    rs, one = edge_one(dev)
     st = fb.forward_with_state(rs, one["means3D"], one["opacities"], shs=one["shs"], scales=one["scales"],
                                rotations=one["rotations"])
     T = ((100 + 15) // 16) * ((60 + 15) // 16)
     assert st["num_rendered"] == T and int(st["radii"][0]) > 0
-    if refdgr.available():
-        ref = refdgr.forward(rs, one["means3D"], one["opacities"], shs=one["shs"], scales=one["scales"], rotations=one["rotations"])
-        assert (st["color"] - ref["color"]).abs().max().item() <= 1e-4
+    check_forward(golden_case("parity_edge_one"), {"color": st["color"]})
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
+def edge_one(device):
+    cam, g, rs = scene(2_000, 100, 60, 2, 1, device, 0.25)
+    one = dict(means3D=torch.tensor([[0.0, 0.0, 3.0]], device=device), opacities=torch.tensor([[0.9]], device=device),
+               scales=torch.full((1, 3), 5.0, device=device), rotations=torch.tensor([[1.0, 0, 0, 0]], device=device),
+               shs=torch.ones(1, 16, 3, device=device))
+    return rs, one
+
+
+def long_tile_scenes(device):
+    from frosting_b200 import scenes
+    cam = scenes.make_camera(64, 48, device=device)
+    rs = scenes.settings_for(cam, 1, device=device)
+    for P in (3_000, 9_000, 60_000):
+        g = scenes.random_gaussians(P, cam, 77, device=device, large_frac=0.0, near_frac=0.0)
+        g["scales"] = g["scales"] * 3.0
+        g["means3D"][: P // 60, :2] *= 0.02          # pile extra splats on the centre tiles
+        yield P, rs, g
+
+
 def test_long_tile_lists_all_sort_classes(cuda_device):
     """Force per-tile lists through the small (<= 2048, static smem), medium (<= 8192, 160 KB dynamic smem) and
     global-memory sort classes (binning.cu)."""
-    dev = cuda_device
-    from frosting_b200 import scenes
-    W, H = 64, 48
-    cam = scenes.make_camera(W, H, device=dev)
-    rs = scenes.settings_for(cam, 1, device=dev)
     covered = set()
-    for P in (3_000, 9_000, 60_000):
-        g = scenes.random_gaussians(P, cam, 77, device=dev, large_frac=0.0, near_frac=0.0)
-        g["scales"] = g["scales"] * 3.0
-        g["means3D"][: P // 60, :2] *= 0.02          # pile extra splats on the centre tiles
-        ref = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    for P, rs, g in long_tile_scenes(cuda_device):
+        case = golden_case(f"parity_long_{P}")
+        check_inputs(case, *(g[k] for k in KEYS))
         st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
         counts = st["tile_count"]
         print(f"P={P}: tile list lengths min {int(counts.min())} max {int(counts.max())}")
         if bool(((counts > 1) & (counts <= 2048)).any()): covered.add("small")
         if bool(((counts > 2048) & (counts <= 8192)).any()): covered.add("medium")
         if bool((counts > 8192).any()): covered.add("global")
-        R = ref["num_rendered"]
-        assert st["num_rendered"] == R
-        assert torch.equal(st["point_list"], refdgr.binning_views(ref["binning"], R)["point_list"]), P
-        assert torch.equal(st["n_contrib"], refdgr.img_views(ref["img"], H, W)["n_contrib"]), P
-        assert (st["color"] - ref["color"]).abs().max().item() <= 1e-4
+        check_forward(case, _fields(st, LIST_FIELDS))
     assert covered == {"small", "medium", "global"}, covered
 
 
-@pytest.mark.skipif(not _ref_available(), reason="oracle/_ref not built")
+def depth_tie_scene(device):
+    from frosting_b200 import scenes
+    P, W, H = 30_000, 160, 128
+    cam = scenes.make_camera(W, H, device=device)
+    g = scenes.random_gaussians(P, cam, 5, device=device, large_frac=0.0, near_frac=0.0)
+    g["means3D"][:, 2] = torch.tensor([3.0, 4.0, 5.0, 4.0], device=device).repeat(P // 4)   # only 3 distinct depths
+    return P, scenes.settings_for(cam, 0, device=device), g
+
+
 def test_equal_depth_ties_follow_gaussian_index(cuda_device):
     """Exact depth ties: the reference's stable radix sort keeps ascending Gaussian index
     (rasterizer_impl.cu:98-108 emission order); our per-tile sort must reproduce it."""
-    dev = cuda_device
-    P, W, H = 30_000, 160, 128
-    from frosting_b200 import scenes
-    cam = scenes.make_camera(W, H, device=dev)
-    g = scenes.random_gaussians(P, cam, 5, device=dev, large_frac=0.0, near_frac=0.0)
-    g["means3D"][:, 2] = torch.tensor([3.0, 4.0, 5.0, 4.0], device=dev).repeat(P // 4)   # only 3 distinct depths
-    rs = scenes.settings_for(cam, 0, device=dev)
-    ref = refdgr.forward(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
+    P, rs, g = depth_tie_scene(cuda_device)
+    case = golden_case("parity_ties")
+    check_inputs(case, *(g[k] for k in KEYS))
     st = fb.forward_with_state(rs, g["means3D"], g["opacities"], shs=g["shs"], scales=g["scales"], rotations=g["rotations"])
-    R = ref["num_rendered"]
-    assert st["num_rendered"] == R
-    assert torch.equal(st["point_list"], refdgr.binning_views(ref["binning"], R)["point_list"])
-    assert torch.equal(st["n_contrib"], refdgr.img_views(ref["img"], H, W)["n_contrib"])
-    assert (st["color"] - ref["color"]).abs().max().item() <= 1e-4
+    check_forward(case, _fields(st, LIST_FIELDS))
 
 
 def test_fused_frosting_attributes_match_torch_chain(cuda_device):
