@@ -475,12 +475,14 @@ preprocess_fwd_kernel(FwdArgs a) {
         }
         if (!shown) keep = false;
         if (keep) {
-            // the SH row (192 B at degree 3) is consumed last, after a chain of dependent loads; start it moving now
-            const char* row = kFrost ? reinterpret_cast<const char*>(a.fr.d_sh_rest + (size_t)idx * a.fr.sh_rest * 3)
-                                     : reinterpret_cast<const char*>(a.in.d_shs + (size_t)idx * a.prm.sh_coeffs * 3);
-            if (kFrost || a.in.d_shs != nullptr) {
+            // the SH row (192 B at degree 3) is consumed last, after a chain of dependent loads; start it moving now.
+            // Frosting mode at sh_rest == 0 has no rest row (NULL pointer): nothing to prefetch.
+            const int row_floats = kFrost ? a.fr.sh_rest * 3 : a.prm.sh_coeffs * 3;
+            const char* row = kFrost ? reinterpret_cast<const char*>(a.fr.d_sh_rest + (size_t)idx * row_floats)
+                                     : reinterpret_cast<const char*>(a.in.d_shs + (size_t)idx * row_floats);
+            if (kFrost ? a.fr.sh_rest > 0 : a.in.d_shs != nullptr) {
                 asm volatile("prefetch.global.L1 [%0];" ::"l"(row));
-                if (a.prm.sh_coeffs * 12 > 128) asm volatile("prefetch.global.L1 [%0];" ::"l"(row + 128));
+                if (row_floats * 4 > 128) asm volatile("prefetch.global.L1 [%0];" ::"l"(row + 128));
             }
         } else if (valid) {
             a.radii[idx] = 0;

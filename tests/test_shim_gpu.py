@@ -238,16 +238,32 @@ def test_frosting_render_equals_the_two_step_path(cuda_device):
         assert float(p1[k].grad[dead].abs().sum()) == 0.0, k
 
 
+# (SH rest coefficients R, degree D): checkpoints trained at degree 0-3 (R = 0, 3, 8, 15), and Frosting's SH warm-up,
+# which renders a degree-3 layout at degree 0, 1, 2 first.  (15, 3) is the full layout.
+FROSTING_SH = [(0, 0), (3, 0), (3, 1), (8, 0), (8, 2), (15, 0), (15, 1), (15, 2), (15, 3)]
+
+
 def test_frosting_mode_equals_the_attribute_kernel_route(cuda_device):
     """Row f1 proper: `frosting_render` (the rasterizer reads the parameters itself, nothing materialised, parameter
     gradients written by the per-Gaussian backward for rendered rows only) against `frosting_render_two_step` (attribute
     kernel -> rasterizer -> attribute backward): bit-identical image and radii, gradients equal up to the order of the
     blend backward's float atomics; the optimizer-sink route gives the same numbers as the autograd route."""
-    dev = cuda_device
+    _frosting_mode_against_the_attribute_kernel_route(cuda_device, 15, 3)
+
+
+@pytest.mark.parametrize("R,D", [rd for rd in FROSTING_SH if rd != (15, 3)])
+def test_frosting_mode_equals_the_attribute_kernel_route_at_lower_sh_layouts(cuda_device, R, D):
+    """The same comparison with fewer rest coefficients per row (R < 15: narrower rows, R = 0: no rest tensor) and at
+    degrees below the row's (D < 3: coefficients past (D + 1)^2 are not read and get zero gradients)."""
+    _frosting_mode_against_the_attribute_kernel_route(cuda_device, R, D)
+
+
+def _frosting_mode_against_the_attribute_kernel_route(dev, R, D):
     for (W, H, P, faces, occl) in ((320, 200, 50_000, 8000, True), (200, 120, 3001, 500, False)):
         cam = scenes.make_camera(W, H, device=dev)
-        params, mesh = scenes.frosting_layer(P, cam, 11, n_faces_target=faces, device=dev, view_distance=4.5)
-        rs = scenes.settings_for(cam, 3, device=dev)
+        params, mesh = scenes.frosting_layer(P, cam, 11, n_faces_target=faces, device=dev, view_distance=4.5,
+                                             sh_coeffs=R + 1)
+        rs = scenes.settings_for(cam, D, device=dev)
         fv = None
         if occl:
             _, fv, _ = fb.rasterize_mesh(mesh["verts"], mesh["faces"], cam.full_proj_transform, H, W, mark_last_on_bg=True)

@@ -23,10 +23,56 @@ def scene(P, W, H, seed, sh_degree, device, bg=0.0):
     return cam, g, rs
 
 
+# ---- float64 statement of the SH colour (computeColorFromSH) ------------------------------------------------------
+SH_C0 = 0.28209479177387814
+SH_C1 = 0.4886025119029199
+SH_C2 = (1.0925484305920792, -1.0925484305920792, 0.31539156525252005, -1.0925484305920792, 0.5462742152960396)
+SH_C3 = (-0.5900435899266435, 2.890611442640554, -0.4570457994644658, 0.3731763325901154, -0.4570457994644658,
+         1.445305721320277, -0.5900435899266435)
+
+
+def sh_layouts():
+    """Every (coefficients per row M, degree D) the plain path accepts: M in {1, 4, 9, 16}, (D + 1)^2 <= M."""
+    return [(M, D) for M in (1, 4, 9, 16) for D in range(4) if (D + 1) ** 2 <= M]
+
+
+def sh_dirs64(means, campos):
+    """Unit view directions (means - campos) / |means - campos| in float64 (differentiable w.r.t. means)."""
+    d = torch.as_tensor(means).double() - torch.as_tensor(campos).double().reshape(1, 3)
+    return d / d.norm(dim=1, keepdim=True)
+
+
+def sh_basis64(dirs, D):
+    """[N, (D+1)^2] real SH basis values at unit directions `dirs` [N, 3], float64, in the coefficient order and sign
+    convention of computeColorFromSH."""
+    x, y, z = dirs[:, 0], dirs[:, 1], dirs[:, 2]
+    b = [torch.full_like(x, SH_C0)]
+    if D > 0:
+        b += [-SH_C1 * y, SH_C1 * z, -SH_C1 * x]
+    if D > 1:
+        xx, yy, zz = x * x, y * y, z * z
+        b += [SH_C2[0] * x * y, SH_C2[1] * y * z, SH_C2[2] * (2 * zz - xx - yy), SH_C2[3] * x * z, SH_C2[4] * (xx - yy)]
+    if D > 2:
+        b += [SH_C3[0] * y * (3 * xx - yy), SH_C3[1] * x * y * z, SH_C3[2] * y * (4 * zz - xx - yy),
+              SH_C3[3] * z * (2 * zz - 3 * xx - 3 * yy), SH_C3[4] * x * (4 * zz - xx - yy), SH_C3[5] * z * (xx - yy),
+              SH_C3[6] * x * (xx - 3 * yy)]
+    return torch.stack(b, 1)
+
+
+def sh_color64(shs, dirs, D):
+    """computeColorFromSH in float64: (colour before the clamp = sum_k b_k(dir) sh_k + 0.5 [N, 3], clamp bits [N, 3]).
+    Only the first (D+1)^2 coefficients of each row are read; the clamped colour is raw.clamp_min(0)."""
+    n = (D + 1) ** 2
+    raw = (sh_basis64(dirs, D)[:, :, None] * torch.as_tensor(shs)[:, :n].double()).sum(1) + 0.5
+    return raw, raw < 0
+
+
 def rel_err_stats(a, b):
     """Gradient tolerance used throughout: error relative to the tensor's scale, plus the fraction of
     significant elements whose own relative error exceeds 1e-3."""
     a, b = a.double().flatten(), b.double().flatten()
+    if b.numel() == 0:                  # e.g. the SH rest gradient of a degree-0 model: [P, 0, 3]
+        return 0.0, 0.0
     scale = b.abs().max().clamp_min(1e-30)
     diff = (a - b).abs()
     max_rel_to_scale = (diff.max() / scale).item()
